@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- ROI-crops/s through iDispNet (cost volume + 28-layer 3-D stack + soft-argmin) on B200.
 
-Contract: `python bench.py --gpus N --steps K --warmup W [--impl reference]`; under torchrun one rank
+Contract: `python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]`; under torchrun one rank
 per GPU.  A step = one pass of the hot path over one batch of synthetic ROI feature pairs
 (BASELINE.json configs[1]: 32 ROI pairs of 112x112x32-ch features, D=48 -> 448x448 disparity, per
 GPU; weak scaling).  Prints ONE JSON line on rank 0.
@@ -282,6 +282,22 @@ def make_model(precision, device):
     return m.to(device).eval()
 
 
+DUMP_BYTES_MAX = 60 * 10**6   # keeps a dump under 64 MB
+
+
+def dump_outputs(out_dir, disp):
+    """Write the disparity maps [B, H, W] of one timed step to out_dir/disparity.npy as float32.  A batch larger than
+    DUMP_BYTES_MAX (weak scaling over many GPUs) is cut to a fixed, seeded choice of whole ROIs, kept in batch order."""
+    import numpy as np
+    d = disp.detach().float().cpu().numpy()
+    per_roi = d[0].nbytes if len(d) else 1
+    if d.nbytes > DUMP_BYTES_MAX:
+        keep = np.sort(np.random.default_rng(0).choice(len(d), DUMP_BYTES_MAX // per_roi, replace=False))
+        d = d[keep]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'disparity.npy'), np.ascontiguousarray(d, dtype=np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -292,7 +308,12 @@ def main():
                     help='fp16x2 (default): split-precision tensor-core mode, meets the 1e-3 parity bar; fp16 / bf16: one-word '
                          'tensor-core modes (faster, 0.07 / 0.4 px from the reference); fp32: SIMT parity mode')
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the disparity maps the last timed step returned to DIR/disparity.npy '
+                         '(float32; inputs and weights are seeded, so two builds can be compared output for output)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
@@ -426,14 +447,17 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
         for _ in range(args.steps):
-            step_device()
-        drain()  # N > 1: the current stream waits for every gather still in flight
+            last = step_device()
+        last = drain() if world > 1 else last  # N > 1: the current stream waits for every gather still in flight
         e1.record(stream)
         torch.cuda.synchronize()
         t = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms_total = t.item()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, last)
+        del last
         launches_per_step = lib.idisp_plan_launches_per_forward(plan) + (GATHER_CHUNKS if world > 1 else 0)
         # ---- roofline leg: the same K steps again with CUDA events between the launches (on the launching stream; the plan
         # then launches eagerly instead of replaying its CUDA graph).  Only the per-kernel durations come from here. ----

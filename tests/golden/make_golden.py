@@ -285,6 +285,12 @@ def gen_roi():
         np.savez_compressed(os.path.join(HERE, f'roialign_{name}.npz'), out=out.numpy(),
                             input_crc=recipe.checksum(inp))
         print(f'roialign {name}: out {tuple(out.shape)}')
+    inp, rois = recipe.make_random_roi_inputs()
+    out = {'input_crc': recipe.checksum(inp), 'rois_crc': recipe.checksum(rois)}
+    for i, (ph, pw, sc, sr) in enumerate(recipe.ROI_RANDOM_CONFIGS):
+        out[f'out{i}'] = ref.roi_align_forward(inp, rois, sc, ph, pw, sr).numpy()
+    np.savez_compressed(os.path.join(HERE, 'roialign_random.npz'), **out)
+    print(f'roialign random: {len(recipe.ROI_RANDOM_CONFIGS)} pooling configs')
 
 
 if __name__ == '__main__':

@@ -211,6 +211,19 @@ ROI_CASES = {
         [0, 0, 0, 93, 65], [0, 80, 50, 120, 90], [0, 92, 64, 94, 66], [0, -10, -10, 4, 4]]),
 }
 
+# fresh random boxes over one input, pooled at several (pooled_h, pooled_w, spatial_scale, sampling_ratio)
+ROI_RANDOM_CONFIGS = [(7, 7, 1.0, 0), (5, 9, 0.5, 2), (16, 16, 1.0, 3)]
+
+
+def make_random_roi_inputs():
+    """[2,5,40,60] input and 12 random boxes (some reach past the border), for golden roialign_random.npz."""
+    g = torch.Generator().manual_seed(5)
+    inp = torch.randn(2, 5, 40, 60, generator=g)
+    xy = torch.rand(12, 2, generator=g) * torch.tensor([50., 30.])
+    wh = torch.rand(12, 2, generator=g) * torch.tensor([40., 30.])
+    rois = torch.cat([torch.randint(0, 2, (12, 1), generator=g).float(), xy, xy + wh], 1)
+    return inp, rois
+
 
 # per-ROI disparity hand-off (disprcnn3d.py:161-190, point_rcnn.py:113-136): integer-expanded boxes inside the image (the
 # detector clips its boxes, structures/bounding_box.py clip_to_image), S x S ROI maps, binary masks, fu*baseline per ROI
