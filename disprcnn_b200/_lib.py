@@ -87,6 +87,9 @@ PROTOTYPES = {
     'idisp_stereo_rois': (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _i, _vp, _vp, _vp, _vp]),
     'idisp_roi_disparity_paste': (_i, [_vp, _i, _i, _vp, _vp, _vp, _i, _vp, _i, _i, _vp, _vp]),
     'idisp_roi_depth_paste': (_i, [_vp, _i, _i, _vp, _vp, _vp, _i, _i, _vp, _vp]),
+    'idisp_roi_points_count': (_i, [_vp, _i, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _f, _i, _vp, _vp]),
+    'idisp_roi_points_choice': (_i, [_i, _i, _vp]),
+    'idisp_roi_points_gather': (_i, [_vp, _i, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _f, _i, _vp, _vp, _i, _f, _vp, _vp, _vp, _vp, _vp]),
     'idisp_cost_volume': (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     'idisp_conv3d': (_i, [_vp, _i, _i, _i, _i, _i, _vp, _i, _i, _vp, _vp, _vp, _i, _i, _vp, _vp]),
     'idisp_softargmin': (_i, [_vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),

@@ -5,39 +5,15 @@
 //     the per-image map is the maximum over the image's ROIs;
 //   * PointRCNN.process_input, modeling/pointnet_module/point_rcnn/lib/net/point_rcnn.py:113-136 -- the same resize + shift, then
 //     depth = fu*baseline / (disp + 1e-6) pasted into a per-ROI image-sized map (which back_project masks and back-projects).
-// Core (structures/disparity.py:39-78, DisparityMap.resize / crop): bilinear align_corners=True resize of the [S,S] map to
-// (h, wmax) with h = y2-y1, wmax = max(x2-x1, x2p-x1p), value * wmax / S (as (v / S) * wmax in float), crop to x2-x1 columns.
+// Core: roi_box / roi_disp_at (roi_box.cuh, shared with roi_points.cu).
 // The reference does this per ROI in Python (.tolist() syncs, one image-sized zeros + interpolate + slice-assign per ROI); here
 // one thread per image pixel walks the ROIs of its image and samples the low-resolution map directly -- nothing image-sized per
 // ROI is materialised in the disparity form.  Integer box arithmetic is exact; the interpolation follows ATen's index math
 // (scale = (in-1)/(out-1), i0 = (int)src, lambda = src - i0) so results agree with the reference to fp32 rounding.
 // Roofline: HBM (writes N*H*W*4 B, reads the touched parts of the R low-resolution maps from L2).
-#include "common.cuh"
+#include "roi_box.cuh"
 
 namespace idisp {
-
-struct RoiBox { int x1, y1, x2, y2, x1p, x2p; };
-
-__device__ __forceinline__ RoiBox roi_box(const float *__restrict__ lb, const float *__restrict__ rb, int r)
-{
-  RoiBox b;   // expand_box_to_integer (utils/stereo_utils.py:219-229): floor the top-left, ceil the bottom-right; NOT clamped
-  b.x1 = (int)floorf(lb[r * 4 + 0]); b.y1 = (int)floorf(lb[r * 4 + 1]); b.x2 = (int)ceilf(lb[r * 4 + 2]); b.y2 = (int)ceilf(lb[r * 4 + 3]);
-  b.x1p = (int)floorf(rb[r * 4 + 0]); b.x2p = (int)ceilf(rb[r * 4 + 2]);
-  return b;
-}
-
-// resized (not yet shifted) disparity of ROI r at image pixel (y, x) inside its box (disparity.py:39-78 as called at disprcnn3d.py:173-175)
-__device__ __forceinline__ float roi_disp_at(const float *__restrict__ d, int S, const RoiBox &b, int y, int x)
-{
-  const int h = b.y2 - b.y1, w = b.x2 - b.x1, wp = b.x2p - b.x1p, wmax = w > wp ? w : wp;
-  const float sh = h > 1 ? (float)(S - 1) / (float)(h - 1) : 0.f, sw = wmax > 1 ? (float)(S - 1) / (float)(wmax - 1) : 0.f;
-  const float fy = sh * (float)(y - b.y1), fx = sw * (float)(x - b.x1);
-  const int y0 = (int)fy, x0 = (int)fx;
-  const int y1 = y0 + (y0 < S - 1 ? 1 : 0), x1 = x0 + (x0 < S - 1 ? 1 : 0);
-  const float ly = fy - (float)y0, lx = fx - (float)x0, hy = 1.f - ly, hx = 1.f - lx;
-  const float v = hy * (hx * __ldg(d + y0 * S + x0) + lx * __ldg(d + y0 * S + x1)) + ly * (hx * __ldg(d + y1 * S + x0) + lx * __ldg(d + y1 * S + x1));
-  return __fmul_rn(__fdiv_rn(v, (float)S), (float)wmax);
-}
 
 // per-image disparity map: out[n][y][x] = max over the image's ROIs of clamp(disp, 0) * mask   (disprcnn3d.py:176-183)
 // roi_start[n] .. roi_start[n+1]: the ROIs of image n (ROIs are grouped by image, as torch.split(output, ...) assumes, :162)

@@ -34,7 +34,8 @@
 extern "C" {
 #endif
 
-#define IDISP_VERSION 2  /* 2: + idisp_extractor_*, idisp_roi_*_paste, idisp_stereo_rois, idisp_plan_forward_host_async / host_wait */
+#define IDISP_VERSION 2  /* 2: + idisp_extractor_*, idisp_roi_*_paste, idisp_stereo_rois, idisp_plan_forward_host_async / host_wait,
+                            idisp_roi_points_count / choice / gather (additions only: every version-2 call is unchanged) */
 
 enum {
   IDISP_OK = 0,
@@ -98,6 +99,36 @@ int idisp_roi_disparity_paste(const float *roi_disp, int R, int S, const float *
                               const int *roi_start, int N, const unsigned char *masks, int H, int W, float *out, void *stream);
 int idisp_roi_depth_paste(const float *roi_disp, int R, int S, const float *left_boxes, const float *right_boxes,
                           const float *fu_baseline, int H, int W, float *out, void *stream);
+
+/* Per-ROI point clouds for PointRCNN (PointRCNN.process_input_eval + back_project(fix_seed=True),
+ * modeling/pointnet_module/point_rcnn/lib/net/point_rcnn.py:189-242 and :37-85): the point-cloud half of SURVEY.md 8f row 3,
+ * without any image-sized map.  Three calls: count (device) -> choice per ROI (host) -> gather (device).
+ * Inputs shared by count and gather (device pointers): roi_disp [R,S,S] f32 (iDispNet's per-ROI disparity), mask_probs [R,M,M] f32
+ * (mask probabilities of the ROI's class), left_boxes / right_boxes [R,4] f32 (x1,y1,x2,y2), image_index [R] int32 (the image
+ * each ROI belongs to), image_wh [n_images][2] int32 (width, height), calib [n_images][7] f64 (fu, fv, cu, cv, tx, ty, fu*b: P2
+ * entries as Calibration defines them, utils/kitti_utils.py:27-67, and Calib.stereo_fuxbaseline), all used as fp32 scalars;
+ * mask_threshold >= 0 and mask_padding >= 1 are the Masker's (modeling/roi_heads/mask_head/inference.py:91-159).
+ *   idisp_roi_points_count: count [R] int32 = n, the number of points of each ROI -- the integer box's pixels inside the pasted
+ *     mask, or, when the mask covers none of them, all of the box's pixels (point_rcnn.py:42-43).  Negative codes: -1 the integer
+ *     box is not inside its image, -2 a depth inside the box is not finite, -3 image_index out of range.
+ *   idisp_roi_points_choice (HOST, no GPU): out [npoints] int32 = the indices numpy draws for n valid points (point_rcnn.py:53-74
+ *     with np.random.seed(0) before each draw), bit for bit: choice(n, P, replace=False) if n > P, else arange(n) followed by
+ *     choice(n, P - n, replace=True); then shuffled.  n >= 1.
+ *   idisp_roi_points_gather: ranks [R,npoints] int32 (device; row r = choice for count[r]) -> pts [R,npoints,3] f32 (rotated about
+ *     y by rot_angle, z clamped at max_depth before the rotation, centred), pts_mean [R,3] f32 (the mean that was subtracted),
+ *     rot_angle [R] f64 (atan2((x1 + x2) / 2 - W0 / 2, fu), W0 = the width of image 0 as in utils/utils_3d.py:88), and -- if
+ *     non-NULL -- pixels [R,npoints] int32 (y * width + x of each point).  A slot whose rank is outside [0, count[r]) (every slot
+ *     of a ROI with count[r] <= 0) gets NaN coordinates and pixel -1.  npoints <= 16384.
+ * R == 0 is a no-op. */
+int idisp_roi_points_count(const float *roi_disp, int R, int S, const float *mask_probs, int M, const float *left_boxes,
+                           const float *right_boxes, const int *image_index, const int *image_wh, const double *calib,
+                           int n_images, float mask_threshold, int mask_padding, int *count, void *stream);
+int idisp_roi_points_choice(int n, int npoints, int *out);
+int idisp_roi_points_gather(const float *roi_disp, int R, int S, const float *mask_probs, int M, const float *left_boxes,
+                            const float *right_boxes, const int *image_index, const int *image_wh, const double *calib,
+                            int n_images, float mask_threshold, int mask_padding, const int *count, const int *ranks,
+                            int npoints, float max_depth, float *pts, float *pts_mean, double *rot_angle, int *pixels,
+                            void *stream);
 
 /* ROIAlign forward.  input [N,C,H,W] f32 NCHW contiguous, rois [R,5] f32
  * (batch_idx,x1,y1,x2,y2), out [R,C,pooled_h,pooled_w] f32 -- all device pointers.
